@@ -2,7 +2,7 @@
 """bench.py -- frames/sec of the per-frame keypoint-voting hot path on synthetic 12288-pt RGB-D clouds.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config linemod|ycb]
-                    [--ms-mode certified|early_exit|strict] [--quick]
+                    [--ms-mode certified|early_exit|strict] [--quick] [--dump-outputs DIR]
 
 Metric / config (BASELINE.json): frames/sec; headline workload = configs[1]: LineMOD-shape synthetic,
 12288 pts, 1 instance, 8 kps, batch 32 per GPU.  A step = one pass of hot path A (Pointnet2MSG.forward)
@@ -309,9 +309,21 @@ class Runner:
     def step_device(self, i):
         d = self.dev_rot[i % self.n_rot]
         nxt = self.dev_rot[(i + 1) % self.n_rot]["cld_rgb_nrm"] if self.lookahead else None
-        poses, _ = self.pipe.run_device(d["cld_rgb_nrm"], d["pcld"], d["labels"], d["ctr_of"], d["kp_of"], next_cloud=nxt)
+        poses, present = self.pipe.run_device(d["cld_rgb_nrm"], d["pcld"], d["labels"], d["ctr_of"], d["kp_of"],
+                                              next_cloud=nxt)
+        self.last = poses, present
         if self.world > 1:   # the single collective of the path: ~1.5 kB per frame
             self.torch.distributed.all_gather_into_tensor(self.gather_buf, poses.reshape(-1))
+
+    def outputs(self, n_feature_points=1024):
+        """What the last device step computed, on the host as float32: poses [B,n_cls,3,4], present [B,n_cls] and hot
+        path A's features [B,128,N] at a fixed seeded sample of n_feature_points points (the poses do not depend on
+        the features: the votes are inputs).  Call right after the step: later steps reuse the output buffers."""
+        poses, present = self.last
+        pts = np.sort(np.random.default_rng(0).choice(self.cfg["n_points"], n_feature_points, replace=False))
+        feats = self.pipe.features.index_select(2, self.torch.from_numpy(pts).to(self.dev))
+        return {"poses": poses.float().cpu().numpy(), "present": present.float().cpu().numpy(),
+                "features_sample": feats.float().cpu().numpy()}
 
     def step_host(self, i):
         self.pipe.run_host(self.host_rot[i % self.n_rot], self.host_rot[(i + 1) % self.n_rot] if self.lookahead else None)
@@ -338,7 +350,7 @@ class Runner:
         ms = e0.elapsed_time(e1)
         return pdist.max_over_ranks(ms, self.dev), (lib.pvn3d_launch_count() - l0 if lib is not None else 0)
 
-    def measure(self, steps, warmup, lib, e2e=True, clocks=True):
+    def measure(self, steps, warmup, lib, e2e=True, clocks=True, keep_outputs=False):
         # W untimed steps of exactly the loop that is timed next (indices -W..-1, so that the look-ahead of the
         # last warm-up step names the first timed batch), then K timed steps; first the device-resident loop,
         # then the same for the host loop
@@ -346,6 +358,7 @@ class Runner:
             self.step_device(i)
         sampler = ClockSampler(self.dev.index or 0).start() if (clocks and self.rank == 0) else None
         ms_dev, launches = self.timed(self.step_device, steps, lib)
+        kept = self.outputs() if keep_outputs else None
         ms_e2e = None
         if e2e:
             for i in range(-warmup, 0):
@@ -355,6 +368,8 @@ class Runner:
         frames = self.B * self.world * steps
         out = {"value": frames / (ms_dev * 1e-3), "unit": "frames/s", "ms_per_step": ms_dev / steps,
                "global_batch": self.B * self.world, "gpu_launches": int(launches), "clocks": ck}
+        if kept is not None:
+            out["outputs"] = kept
         if e2e:
             out["e2e"] = {"value": frames / (ms_e2e * 1e-3), "unit": "frames/s", "h2d_bytes_per_step": self.pipe.h2d_bytes(),
                           "d2h_bytes_per_step": self.pipe.d2h_bytes(), "ms_per_step": ms_e2e / steps}
@@ -545,7 +560,11 @@ def b200_arm(args, json_out):
 
     la = not args.no_lookahead
     run = Runner(torch, cfg, dev, rank, world, args.ms_mode, overlap=overlap, engine=args.engine, lookahead=la)
-    head = run.measure(args.steps, args.warmup, lib)
+    head = run.measure(args.steps, args.warmup, lib, keep_outputs=bool(args.dump_outputs) and rank == 0)
+    if "outputs" in head:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in head.pop("outputs").items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
     B = run.B
     line = None
     if rank == 0:
@@ -723,7 +742,9 @@ def b200_arm(args, json_out):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps K of the headline loop (the frames/s value and e2e); without --quick the other "
+                         "loops run max(3, K/2) steps (other mean-shift modes), max(5, K/2) (YCB) and max(3, K/4) (stress)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="linemod", choices=["linemod", "ycb"])
@@ -735,7 +756,14 @@ def main():
     ap.add_argument("--quick", action="store_true", help="headline + stage split only (development runs, ncu)")
     ap.add_argument("--engine", default="fused", choices=["fused", "modules"],
                     help="hot path A: fused tcgen05 engine (default) or module graph with cuDNN/cuBLAS MLPs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, float32: poses, present "
+                         "and a fixed seeded sample of 1024 points of the [B,128,N] features (16 MB at batch 32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path: it needs --impl b200")
     # stdout carries exactly ONE line (the JSON): everything any library prints to fd 1 from here on
     # (NCCL prints its version there) goes to stderr; the JSON is written to the saved descriptor
     sys.stdout.flush()

@@ -1125,7 +1125,11 @@ __global__ void __launch_bounds__(kMsThreads, 3) ms_iterate_kernel(MsArgs a) {
         const unsigned *vw = a.viol + static_cast<size_t>(f) * a.viol_words;
         for (int it = prev_lo; it <= prev_hi; ++it)
           if (!((vw[it >> 5] >> (it & 31)) & 1u)) { tz = it; break; }
-        const int s = a.star_it[f];
+        // CTAs that are through with these decisions already run tiles of phase p, which may set star_it
+        // to an iteration of phase p; only a value from a finished phase keeps the decision identical in
+        // every CTA (a CTA that alone closed the fit could leave the loop while the others wait at the barrier)
+        int s = a.star_it[f];
+        if (s > prev_hi) s = 0;
         int T = 0;
         if (tz) T = (early && s > 0 && s < tz) ? s : tz;
         else if (early && s > 0) T = s;

@@ -1,4 +1,5 @@
 """Shared helpers of the GPU parity tests (test infrastructure)."""
+import hashlib
 import importlib.util
 import os
 
@@ -12,6 +13,36 @@ _ref_tried = False
 # (n -> m, radii, nsamples) of the four SA levels (reference pvn3d.py:65-111)
 SA_LEVELS = [(12288, 2048, (0.0175, 0.025), (16, 32)), (2048, 1024, (0.025, 0.05), (16, 32)),
              (1024, 512, (0.05, 0.1), (16, 32)), (512, 128, (0.1, 0.2), (16, 32))]
+# (batch, points) of the DenseFusion + heads parity cases (tests/test_heads_gpu.py)
+HEADS_CASES = [(2, 2048), (1, 12288), (2, 1000)]
+
+
+def digest(a) -> str:
+    """SHA-256 of an array's dtype, shape and bytes: the stored form of reference outputs too large to keep."""
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()
+
+
+def state_dict_digest(module) -> str:
+    h = hashlib.sha256()
+    for k, v in module.state_dict().items():
+        h.update(k.encode())
+        h.update(digest(v.detach().cpu().numpy()).encode())
+    return h.hexdigest()
+
+
+def sample(a, k, rows=False, seed=0):
+    """A fixed, seeded sample of k elements of `a` (flattened), or of k rows of a 2-D `a`, in storage order."""
+    a = np.asarray(a)
+    n = a.shape[0] if rows else a.size
+    pos = np.sort(np.random.default_rng(seed).choice(n, size=min(k, n), replace=False))
+    return a[pos] if rows else a.reshape(-1)[pos]
+
+
+def sa_autograd_inputs():
+    """xyz [2,512,3] and features [2,6,512] of the SA-module gradient parity test"""
+    return (np.random.default_rng(1).uniform(size=(2, 512, 3)).astype(np.float32),
+            np.random.default_rng(3).uniform(size=(2, 6, 512)).astype(np.float32))
 
 
 def load_ref_ext():

@@ -110,26 +110,42 @@ def test_frame_shard_and_gather_gloo_world2(n_frames):
     assert all(ok for _, ok, _ in res) and all(mx == 2.0 for _, _, mx in res)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/pvn3d"), reason="reference checkout not present")
-def test_unmodified_reference_binds_to_the_drop_in():
+def test_unmodified_reference_binds_to_the_drop_in(tmp_path):
     """`from lib.pointnet2_utils import _ext` (reference pointnet2_utils.py:19) resolves to this package's
-    module, and the post-processing names are rebound -- run in a subprocess to keep sys.modules clean."""
+    module, and the post-processing names are rebound -- on a stand-in tree with the reference's module paths and
+    the import lines compat.install() relies on, in a subprocess to keep sys.modules clean.  The stand-in does not
+    import what the real lib/ imports, so the shims for it (torch._six, yaml.load's Loader, neupeak / plyfile / pcl)
+    are exercised here only through test_compat_install_registers_ext_module; importing the real reference Python
+    and running its Pointnet2MSG, SA autograd and cal_frame_poses on the drop-in is done by
+    tests/golden/make_golden_ref_gpu.py when the reference outputs are recorded.  The "CPU not supported" check runs
+    through this package's mirror Pointnet2MSG, which calls the same `_ext` entry points."""
     import subprocess
+    tree = {
+        "lib/pointnet2_utils/pointnet2_utils.py": "from lib.pointnet2_utils import _ext\n",
+        "lib/utils/meanshift_pytorch.py": "class MeanShiftTorch:\n    pass\n",
+        "lib/utils/pvn3d_eval_utils.py": ("from lib.utils.meanshift_pytorch import MeanShiftTorch\n"
+                                          "def cal_frame_poses(*args):\n    pass\n"
+                                          "def cal_frame_poses_lm(*args):\n    pass\n"),
+    }
+    for rel, text in tree.items():
+        (tmp_path / rel).parent.mkdir(parents=True, exist_ok=True)
+        (tmp_path / rel).write_text(text)
     code = (
         "import sys; sys.path.insert(0, %r)\n"
-        "from pvn3d_b200 import compat, _ext, meanshift\n"
-        "compat.install('/root/reference/pvn3d', patch_post=True)\n"
+        "from pvn3d_b200 import compat, _ext, eval_utils, meanshift\n"
+        "compat.install(%r, patch_post=True)\n"
         "from lib.pointnet2_utils import pointnet2_utils as pu\n"
         "from lib.utils import pvn3d_eval_utils as ev, meanshift_pytorch as ms\n"
-        "from lib.pvn3d import Pointnet2MSG\n"
+        "from pvn3d_b200.pointnet2 import Pointnet2MSG\n"
         "import torch\n"
         "assert pu._ext is _ext and ms.MeanShiftTorch is meanshift.MeanShiftTorch\n"
-        "assert ev.cal_frame_poses.__module__ == 'pvn3d_b200.eval_utils'\n"
+        "assert ev.MeanShiftTorch is meanshift.MeanShiftTorch\n"
+        "assert ev.cal_frame_poses is eval_utils.cal_frame_poses and ev.cal_frame_poses_lm is eval_utils.cal_frame_poses_lm\n"
         "m = Pointnet2MSG(input_channels=6)\n"
         "try:\n    m(torch.zeros(1, 4096, 9)); raise SystemExit(3)\n"
         "except RuntimeError as e:\n    assert 'CPU not supported' in str(e)\n"
-        "print('ok')\n") % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
+        "print('ok')\n") % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))), str(tmp_path))
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=tmp_path)
     assert r.returncode == 0 and "ok" in r.stdout, r.stderr[-2000:]
 
 

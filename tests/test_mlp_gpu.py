@@ -124,20 +124,35 @@ def test_fp_first_layer_fuses_interpolation(cuda_dev):
     d2, nn = pn2.three_nn(unk, kn)
     kf = torch.from_numpy(rng.normal(size=(b_, m_k, c2)).astype(np.float32))
     sk = torch.from_numpy(rng.normal(size=(b_, n_u, c1)).astype(np.float32))
-    nw = mlp.three_nn_weights(torch.from_numpy(d2).to(cuda_dev))
+    d2_dev = torch.from_numpy(d2).to(cuda_dev)
+    nw = mlp.three_nn_weights(d2_dev)
+    # nn_weights_kernel in exactly rounded fp32, its order of operations: r_i = 1 / (sqrt(d_i) + 1e-8),
+    # w_i = r_i / ((r_1 + r_2) + r_3) -- the same bits on every host
+    r = np.float32(1) / (np.sqrt(d2) + np.float32(1e-8))
+    w_exact = r / ((r[..., 0] + r[..., 1]) + r[..., 2])[..., None]
+    nw_h = nw.cpu().numpy()
+    assert np.array_equal(nw_h, w_exact), f"{int((nw_h != w_exact).sum())} weights differ, max {np.abs(nw_h - w_exact).max():.3e}"
     dr = 1.0 / (torch.sqrt(torch.from_numpy(d2)) + 1e-8)                        # pointnet2_modules.py:184-186
     wref = dr / dr.sum(2, keepdim=True)
-    assert (nw.cpu() - wref).abs().max() < 2e-7
+    # torch's CPU kernels round the reciprocal and the sum their own way (1 ulp here): a float tolerance
+    assert (torch.from_numpy(nw_h) - wref).abs().max() < 2e-7
     interp = (kf[torch.arange(b_)[:, None, None], torch.from_numpy(nn).long()] * wref[..., None]).sum(2)
     X = torch.cat([interp, sk], -1).reshape(-1, c2 + c1)
     w = torch.from_numpy((rng.normal(size=(128, c2 + c1)) / 16).astype(np.float32))
     bias = torch.from_numpy(rng.normal(size=128).astype(np.float32))
     want = ref_dense(mlp.tf32_round(X), mlp.tf32_round(w), bias, True, 0)
     layer = mlp.PackedLayer(w.to(cuda_dev), bias.to(cuda_dev))
-    skd = sk.to(cuda_dev)
-    out = mlp.mlp_fp_first(kf.to(cuda_dev), torch.from_numpy(nn).to(cuda_dev), nw, skd.data_ptr(), c1, c1, layer).cpu()
+    kfd, nnd, skd = kf.to(cuda_dev), torch.from_numpy(nn).to(cuda_dev), sk.to(cuda_dev)
+    out = mlp.mlp_fp_first(kfd, nnd, nw, skd.data_ptr(), c1, c1, layer).cpu()
+    # same inputs, same bits: the producers' K chunks, the weight stages and the accumulators leave nothing to chance
+    again = mlp.mlp_fp_first(kfd, nnd, nw, skd.data_ptr(), c1, c1, layer).cpu()
+    diff = (out != again).nonzero()
+    assert diff.numel() == 0, f"second launch differs in rows {diff[:, 0].unique()[:8].tolist()}, columns {diff[:, 1].unique()[:8].tolist()}"
     # interpolation rounds to TF32 after a 3-term fp32 sum: allow one TF32 ulp of the operands
-    assert (out[:, :128] - want).abs().max() <= 1e-3 * want.abs().max()
+    err = (out[:, :128] - want).abs()
+    bad = (err > 1e-3 * want.abs().max()).nonzero()
+    assert bad.numel() == 0, (f"max error {float(err.max()):.3e} vs bound {1e-3 * float(want.abs().max()):.3e}, rows "
+                              f"{bad[:, 0].unique()[:8].tolist()}, columns {bad[:, 1].unique()[:8].tolist()}")
 
 
 def test_fused_pointnet2msg_matches_reference_features(cuda_dev, golden_dir):
